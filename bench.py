@@ -5,7 +5,7 @@ One "step" = one pass of the hot path (the fused OSC kernel: chain walk -> J, M,
 one batch of B synthetic joint states per GPU (B = 65 536, fp64: the UR5 configuration of BASELINE.json,
 configs[1], driven through OSC.generate with use_C so that {J, M, g, c_forces} are all on the path).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path (one JSON line on rank 0)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # our CUDA path (one JSON line on rank 0)
   python bench.py --impl reference [...]                         # the reference's CPU path on the host cores
 
 Under torchrun (N > 1) every rank owns its own B states (weak scaling, no data-path collective in the timed step);
@@ -26,6 +26,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 
 METRIC = "OSC control evals/sec (batched UR5 6-DOF)"
@@ -435,6 +436,10 @@ def run_ours(args):
     t = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
     clocks = sampler.stop() if sampler else None
     value = world * B * args.steps / t
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path received in its last step: u of rank 0's batch (B x 6 float64, 3 MB)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "u.npy"), outs[(args.steps - 1) % n_sets].cpu().numpy())
 
     # ---- the one collective of the path (BASELINE config 5 / SURVEY S8e): all-gather of u so that every rank holds the
     #      (world * B, n) array.  Measured three ways with device events, max over ranks: NCCL all-gather alone, the
@@ -742,8 +747,13 @@ def main():
     ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the CUDA path, write the control output u of its last step as "
+                         "DIR/u.npy (float64); the inputs are seeded, so two builds can be compared output for output")
     ap.add_argument("--as-shipped-worker", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.as_shipped_worker:
         as_shipped_worker(args.as_shipped_worker)
     elif args.impl == "reference":

@@ -4,8 +4,8 @@ MuJoCo is not in this image, so the importer cannot be compared with ``MujocoCon
 "parity unpinned").  It is checked (i) by a round trip: a random serial chain is written out as MJCF (body pos/quat,
 joint pos/axis, inertial pos/quat/mass/diaginertia, an EE body) and read back — the oracle built from the imported
 descriptor must reproduce, for random joint angles, the world poses computed directly from the numbers that went into
-the file; (ii) on the reference's own ``ur5.xml`` where it is available (development container): the zero pose is the
-sum of the body offsets in the file, and each joint moves the end effector about the axis the file names.
+the file; (ii) on the reference's own UR5 model (tests/golden/ur5_mjcf.xml: its ``ur5.xml`` without geometry): the zero
+pose is the sum of the body offsets in the file, and each joint moves the end effector about the axis the file names.
 """
 import os
 
@@ -102,10 +102,9 @@ def test_round_trip_through_an_mjcf_file(tmp_path, n):
     assert np.allclose(li[1:, 0], [b["mass"] for b in bodies]) and np.allclose(li[1:, 3:], [b["di"] for b in bodies])
 
 
-UR5_XML = "/root/reference/abr_control/arms/ur5/ur5.xml"
+UR5_XML = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ur5_mjcf.xml")
 
 
-@pytest.mark.skipif(not os.path.exists(UR5_XML), reason="the reference checkout is only present in the development container")
 def test_reference_ur5_xml():
     desc = chain_desc_from_mjcf(UR5_XML)
     assert desc["n_joints"] == 6 and desc["joint_names"] == [f"joint{i}" for i in range(6)]
